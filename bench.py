@@ -18,6 +18,9 @@ pinned-host -> device copy of the images and the device -> host copy of every pr
 `--impl reference` times the reference algorithm's CPU implementation (the oracle port, all host threads) on a
 bounded sample of the same workload: `--ref-views` (default 1) of the views per step at the same resolution - its
 `config` says so (`views_per_step`), its global attention spans that many views only.
+
+`--dump-outputs DIR` writes the predictions of the last timed step as DIR/<name>.npy (see `dump_outputs`).  Weights
+and images are seeded, so two builds run with the same arguments can be compared array by array.
 """
 import argparse
 import json
@@ -31,11 +34,13 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 METRIC = "views/sec (518^2, V=8)"
 TENSOR_OPS = ("iggt_gemm_store16", "iggt_gemm_store32", "iggt_gemm_resid32", "iggt_gemm_qkv", "iggt_conv_nhwc",
               "iggt_attention_fwd")
+DUMP_BYTES = 64 * 10 ** 6
 
 
 # ------------------------------------------------------------------------------------------- helpers
@@ -93,6 +98,25 @@ class ClockSampler:
                 "samples": len(sm)}
 
 
+def dump_outputs(out, path):
+    """Writes the prediction dict `out` as `path`/<name>.npy in float32: every key a caller receives except `images`
+    (the caller's own input handed back); `pose_enc`, one [B, S, 9] tensor per camera-head iteration, is stacked to
+    [iters, B, S, 9].  If the arrays exceed DUMP_BYTES in all, each one is written as the same fraction of its
+    elements: a 1-D array of the values at sorted flat positions drawn with a fixed seed, the same for every run."""
+    arrays = {k: (torch.stack(v) if isinstance(v, list) else v).detach().float().cpu()
+              for k, v in out.items() if k != "images"}
+    total = sum(a.numel() * 4 for a in arrays.values())
+    os.makedirs(path, exist_ok=True)
+    for name, a in sorted(arrays.items()):
+        if total > DUMP_BYTES:
+            keep = a.numel() * DUMP_BYTES // total
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, name + ".npy"), a.numpy())
+    print(f"[bench] {len(arrays)} outputs of the last timed step -> {path}"
+          f"{f' (a sample of {total} bytes)' if total > DUMP_BYTES else ''}", file=sys.stderr)
+
+
 def dist_setup(n_gpus):
     import torch.distributed as dist
     rank = int(os.environ.get("RANK", "0"))
@@ -120,10 +144,12 @@ def run_reference(args):
     times = []
     for i in range(args.warmup + args.steps):
         t0 = time.perf_counter()
-        ref_model.forward(sd, images, model="vggt", skip_part=True, frames_chunk=2)
+        out = ref_model.forward(sd, images, model="vggt", skip_part=True, frames_chunk=2)
         dt = time.perf_counter() - t0
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(out, args.dump_outputs)
     ms = 1e3 * sum(times) / len(times)
     v = S / (ms / 1e3)
     sample = (f"{S} of {args.views} views at {args.size}x{args.size} per step, fp32, same heads "
@@ -157,6 +183,8 @@ def workload_config(args, world):
 def run_b200(args):
     import torch.distributed as dist
     rank, world, local = dist_setup(args.gpus)
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of one process: run it with --gpus 1")
     dev = torch.device("cuda", local)
     torch.cuda.set_device(dev)
     from iggt_official_b200 import ops
@@ -202,6 +230,8 @@ def run_b200(args):
         for _ in range(args.steps):
             out = step(images_dev)
         barrier()
+        if args.dump_outputs:
+            dump_outputs(out, args.dump_outputs)
         if rank == 0:
             print(json.dumps({"quick": True, "launches_per_step": ops.STATS["launches"] // (args.warmup + args.steps)}))
         _finish(world)
@@ -219,6 +249,8 @@ def run_b200(args):
         out = step(images_dev)
     e1.record()
     barrier()
+    if args.dump_outputs:                          # before later replays overwrite the graph's output buffers
+        dump_outputs(out, args.dump_outputs)
     ms = e0.elapsed_time(e1) / args.steps
     launches = (ops.STATS["launches"] - launches0) // args.steps
     if graphed:                                    # replays bypass the Python counter: count one eager forward
@@ -426,7 +458,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch kernels eagerly instead of replaying a CUDA graph")
     ap.add_argument("--quick", action="store_true", help="profiling mode: warm-up + steps only (run this under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -22,6 +22,15 @@ CASES = [
     ("vggt_s2_42x42_stress", "VGGT", 1, 2, 42, 42, "stress", 2, 13),
     ("iggt_s1_56x84_stress", "IGGT", 1, 1, 56, 84, "stress", 3, 14),
 ]
+# tokens4 / tokens23 are [B, S, T, 2048] fp32; beyond this many B*S*T rows a fixture keeps a seeded sample of rows
+# (`token_rows`, indices into the flattened rows) so that it stays under 1 MB.  The prediction heads are kept whole.
+MAX_TOKEN_ROWS = 32
+
+
+def token_rows(n, seed):
+    if n <= MAX_TOKEN_ROWS:
+        return None
+    return torch.randperm(n, generator=torch.Generator().manual_seed(seed))[:MAX_TOKEN_ROWS].sort().values
 
 
 def main():
@@ -53,6 +62,11 @@ def main():
         hook.remove()
         rec = {"case": dict(name=name, model=cls, B=B, S=S, H=H, W=W, kind=kind, wseed=wseed, iseed=iseed),
                "tokens4": toks[4], "tokens23": toks[23]}
+        rows = token_rows(toks[4][..., 0].numel(), iseed)
+        if rows is not None:
+            rec["token_rows"] = rows
+            for i in (4, 23):
+                rec[f"tokens{i}"] = toks[i].flatten(0, -2)[rows].clone()
         for k, v in out.items():
             if k == "images":
                 continue

@@ -1,10 +1,13 @@
-"""Generates tests/golden/preprocess/*.png and tests/golden/preprocess_ref.npz by running the UNMODIFIED reference
+"""Generates tests/golden/preprocess/*.png and tests/golden/preprocess_ref.json by running the UNMODIFIED reference
 `iggt.utils.load_fn.load_and_preprocess_images` (it only needs torch, Pillow and torchvision, all present here) on
-small synthetic views.  Outputs are stored as round(x * 255) uint8 (ToTensor's x / 255 is exactly invertible).
+small synthetic views.  Each output is recorded as its shape and the SHA-256 of round(x * 255) in uint8 (ToTensor's
+x / 255 is exactly invertible, so the digest pins every value bit for bit; the arrays themselves run to megabytes).
 
     python oracle/make_golden_preprocess.py        # needs /root/reference; the fixtures are committed
 """
+import hashlib
 import importlib.util
+import json
 import os
 import sys
 
@@ -43,7 +46,7 @@ def main():
     ref = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(ref)
     os.makedirs(OUT, exist_ok=True)
-    arrays = {}
+    digests = {}
     for name, (mode, size, files) in CASES.items():
         paths = []
         for fn, h, w, seed, alpha in files:
@@ -53,9 +56,16 @@ def main():
         out = ref.load_and_preprocess_images(paths, mode=mode, resize_target_size=size)
         q = (out * 255).round().to(dtype=__import__("torch").uint8)
         assert (q.float().div(255) == out).all()
-        arrays[name] = q.numpy()
+        digests[name] = digest_u8(q.numpy())
         print(name, tuple(out.shape))
-    np.savez_compressed(os.path.join(ROOT, "tests", "golden", "preprocess_ref.npz"), **arrays)
+    with open(os.path.join(ROOT, "tests", "golden", "preprocess_ref.json"), "w") as f:
+        json.dump(digests, f, indent=1)
+
+
+def digest_u8(q):
+    """shape and SHA-256 of a C-ordered uint8 array"""
+    assert q.dtype == np.uint8, q.dtype
+    return {"shape": list(q.shape), "sha256_u8": hashlib.sha256(np.ascontiguousarray(q).tobytes()).hexdigest()}
 
 
 if __name__ == "__main__":

@@ -5,7 +5,7 @@ dependency of the reference, Pillow (`img.resize(size, Image.Resampling.BICUBIC)
 image): `resize_bicubic_u8` restates its published 8-bit algorithm (src/libImaging/Resample.c: bicubic_filter,
 precompute_coeffs, normalize_coeffs_8bpc, ImagingResampleHorizontal_8bpc / Vertical_8bpc) with scalar Python loops for
 the taps and integer numpy for the accumulation.  Pinned by tests/test_preprocess.py against Pillow itself and against
-tests/golden/preprocess_ref.npz, which oracle/make_golden_preprocess.py produced by running the unmodified reference
+tests/golden/preprocess_ref.json, which oracle/make_golden_preprocess.py produced by running the unmodified reference
 function.  Nothing outside tests/, smoke() and bench.py's CPU legs may import this module."""
 import math
 

@@ -29,9 +29,12 @@ def test_oracle_matches_reference(path):
     g = torch.Generator().manual_seed(c["iseed"])
     images = torch.rand(c["B"], c["S"], 3, c["H"], c["W"], generator=g)
     toks = ref_model.aggregator(sd, images)
-    # fp32 vs fp32, different op order only: 5e-5 of the tensor's max magnitude
-    assert _rel(toks[4], rec["tokens4"]) < 5e-5
-    assert _rel(toks[23], rec["tokens23"]) < 5e-5
+    rows = rec.get("token_rows")           # a seeded sample of the B*S*T token rows, in fixtures of many views
+    for i in (4, 23):
+        got = toks[i] if rows is None else toks[i].flatten(0, -2)[rows]
+        # fp32 vs fp32, different op order only: 5e-5 of the tensor's max magnitude
+        assert got.shape == rec[f"tokens{i}"].shape
+        assert _rel(got, rec[f"tokens{i}"]) < 5e-5
     out = ref_model.forward(sd, images, model="iggt" if c["model"] == "IGGT" else "vggt", frames_chunk=2)
     pose = torch.stack(out["pose_enc"], 0)
     assert _rel(pose, rec["pose_enc"]) < 1e-4

@@ -4,6 +4,7 @@ CPU: the oracle restatement is pinned against Pillow itself and against fixtures
 `load_and_preprocess_images` (oracle/make_golden_preprocess.py); the product's host-side tap tables are checked against
 the oracle's.  GPU: the C-ABI kernels must reproduce the fixtures BIT-EXACTLY (byte / integer work)."""
 import glob
+import json
 import os
 import sys
 
@@ -15,12 +16,20 @@ from PIL import Image
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from oracle import ref_preprocess as R                                      # noqa: E402
-from oracle.make_golden_preprocess import CASES, synthetic                  # noqa: E402
+from oracle.make_golden_preprocess import CASES, digest_u8, synthetic       # noqa: E402
 from iggt_official_b200.utils import load_fn                                # noqa: E402
 
 GOLD = os.path.join(ROOT, "tests", "golden")
 RAGGED = [(37, 53, 14, 28), (120, 213, 518, 294), (64, 64, 64, 64), (50, 20, 20, 50), (9, 300, 301, 7),
           (200, 3, 5, 70), (1, 1, 4, 4), (33, 47, 47, 33)]              # (h, w, new_w, new_h)
+
+
+def _assert_equals_reference_fixture(x, name):
+    """x (float32 ndarray) equals the reference's output bit for bit: every value is some k / 255 exactly, and the
+    bytes k have the reference's shape and SHA-256."""
+    q = np.rint(x * np.float32(255)).astype(np.uint8)
+    assert np.array_equal(q.astype(np.float32) / np.float32(255), x)
+    assert digest_u8(q) == json.load(open(os.path.join(GOLD, "preprocess_ref.json")))[name]
 
 
 def _decode(path):
@@ -39,11 +48,10 @@ def test_oracle_resize_matches_pillow(h, w, nw, nh):
 
 @pytest.mark.parametrize("name", sorted(CASES))
 def test_oracle_matches_reference_fixture(name):
-    gold = np.load(os.path.join(GOLD, "preprocess_ref.npz"))[name]
     mode, size, files = CASES[name]
     got = R.load_and_preprocess([_decode(os.path.join(GOLD, "preprocess", f[0])) for f in files], mode, size)
-    assert got.shape == gold.shape
-    assert np.array_equal(got, gold.astype(np.float32) / np.float32(255))
+    assert got.dtype == np.float32
+    _assert_equals_reference_fixture(got, name)
 
 
 @pytest.mark.parametrize("n_in,n_out", [(213, 518), (120, 294), (500, 70), (30, 70), (64, 64), (1, 4), (4000, 518), (7, 3)])
@@ -78,12 +86,11 @@ def test_argument_errors_match_reference():
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", sorted(CASES))
 def test_device_matches_reference_fixture(name):
-    gold = np.load(os.path.join(GOLD, "preprocess_ref.npz"))[name]
     mode, size, files = CASES[name]
     out = load_fn.load_and_preprocess_images([os.path.join(GOLD, "preprocess", f[0]) for f in files], mode=mode,
                                              resize_target_size=size)
-    assert out.is_cuda and out.dtype == torch.float32 and tuple(out.shape) == gold.shape
-    assert torch.equal(out.cpu(), torch.from_numpy(gold).float().div(255))
+    assert out.is_cuda and out.dtype == torch.float32
+    _assert_equals_reference_fixture(out.cpu().numpy(), name)
 
 
 @pytest.mark.gpu
